@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W [--workload autorally|cartpole|double_integrator_tube]
     python bench.py --impl reference ...      # the reference's CPU step() loop (oracle port) on the host cores
     python bench.py --all-configs             # one JSON line per BASELINE config C2..C5 (the last line is the headline C4)
+    python bench.py --dump-outputs DIR ...    # also save what the last timed solve returned, as DIR/<workload>_<array>.npy
 
 A "step" is one optimisation iteration of Controller::computeControl (noise draw -> N x T rollout -> baseline /
 exp-weights -> weighted control average) on synthetic inputs (SURVEY.md §8d). Default workload = the configuration the
@@ -23,13 +24,14 @@ Reported numbers
             and kernels compiled for sm_100 with an Eigen stand-in, "reference kernels, shimmed host") timed on the same
             box for C2 / C4: computeControl Hz with steady_clock around the host call, best of a few rollout block shapes.
   parity_ok (N > 1) the sharded solve against a single-GPU solve of the same seed, checked inside the warm-up.
-The timed regions always cover >= 100 ms of work: `steps` solves are repeated `inner_repeats` times back to back and the
-per-solve mean is reported (a 20-step run of a 0.2 ms solve would otherwise be a 4 ms measurement).
+Each timed region is exactly `steps` solves and the per-solve mean is reported; pick `steps` so that a region covers
+>= 100 ms of work, or the number measures launch overhead and clock noise as much as the solve. How many solves come
+before the last timed one depends only on the arguments, so with the same arguments the outputs saved by --dump-outputs
+are comparable run to run and build to build.
 """
 import argparse
 import ctypes
 import json
-import math
 import os
 import sys
 import threading
@@ -222,6 +224,17 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def _dump_outputs(out_dir, w, U, stats):
+    """What the last timed solve handed its caller: the optimal control sequence U [D][T][C] and, per distribution, the
+    baseline (minimum sample cost), the normaliser (sum of the weights) and the sum of the squared weights."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"U": np.asarray(U, np.float32)}
+    for i, key in enumerate(("baseline", "normalizer", "sum_w2")):
+        arrays[key] = np.array([s[i] for s in stats], np.float32)
+    for key, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{w.name}_{key}.npy"), a)
+
+
 def _base_config(w):
     """The keys both arms (--impl ours / reference) print under `config`, so that the driver's same-config check passes."""
     return {"workload": w.name, "num_rollouts": w.N, "num_timesteps": w.T, "controller": w.controller}
@@ -329,46 +342,25 @@ def run_engine(args, ctx, emit=True, extra=None):
                            "U 2e-5 of the control scale, on every rank"}
         e.seed(w.seed, 0)
 
-    # ---- warm-up + per-solve estimate (sizes the timed regions to >= 100 ms) ------------------------------------------
-    for _ in range(max(args.warmup, 3)):
-        e.solve_into(x0, U, U_out, stats, w.optimization_stride, 0)
-    barrier()
-    t0 = time.perf_counter()
-    for _ in range(10):
-        e.solve_async(x0, U, w.optimization_stride, 0)
-    e.solve_wait()
-    torch.cuda.synchronize()
-    est = (time.perf_counter() - t0) / 10
-    inner = max(1, int(math.ceil(0.14 / max(args.steps * est, 1e-9))))  # >= 100 ms timed, with margin: est includes launch gaps
-    if dist is not None:
-        ti = torch.tensor([inner], device="cuda", dtype=torch.int64)
-        dist.all_reduce(ti, op=dist.ReduceOp.MAX)
-        inner = int(ti.item())
-    n_timed = args.steps * inner
-
+    # ---- warm-up, right before the timed solves (NVML start-up would otherwise leave the GPU idle in between) -------------
     sampler = ClockSampler(local_rank)
     sampler.start()
+    for _ in range(max(args.warmup, 3)):
+        e.solve_into(x0, U, U_out, stats, w.optimization_stride, 0)
+    n_timed = args.steps
 
     # ---- value: solves enqueued back to back, inputs resident (kernel parameter bank), device-timed ---------------------
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    for _attempt in range(3):
-        barrier()
-        ev0.record(stream)
-        for _ in range(n_timed):
-            e.solve_async(x0, U, w.optimization_stride, 0)
-        ev1.record(stream)
-        e.solve_wait()
-        barrier()
-        dev_ms = ev0.elapsed_time(ev1)
-        lo_ms = dev_ms
-        if dist is not None:
-            tm = torch.tensor([dev_ms], device="cuda", dtype=torch.float64)
-            dist.all_reduce(tm, op=dist.ReduceOp.MIN)
-            lo_ms = float(tm.item())
-        if lo_ms >= 100.0:
-            break
-        inner = int(math.ceil(inner * 125.0 / max(lo_ms, 1.0)))  # the estimate was short: enlarge and measure again
-        n_timed = args.steps * inner
+    barrier()
+    ev0.record(stream)
+    for _ in range(n_timed):
+        e.solve_async(x0, U, w.optimization_stride, 0)
+    ev1.record(stream)
+    U_last, stats_last = e.solve_wait()
+    barrier()
+    dev_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        _dump_outputs(args.dump_outputs, w, U_last, stats_last)
 
     # ---- e2e: what Controller::computeControl does per call (mppi_controller.cu:151-241): one blocking C-ABI solve with
     # host buffers, then the host tail on the result — Savitzky-Golay smoothing and the nominal state/output roll-forward
@@ -526,7 +518,7 @@ def run_engine(args, ctx, emit=True, extra=None):
             "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": _base_config(w),
             "engine": {"parallelism": f"rollout-sharded dp{world}", "rollouts_per_gpu": n_local, "k1_launch": info,
-                       "inner_repeats": inner, "timed_solves": n_timed, "timed_ms": dev_ms,
+                       "timed_solves": n_timed, "timed_ms": dev_ms,
                        **_k1_variant(w),
                        "l2": "noise buffer is regenerated on the device every solve (K0 -> K1 through L2/HBM); no data "
                              "is reused across solves; the roofline pass flushes L2 (256 MiB memset) between K0 and K1"},
@@ -588,6 +580,9 @@ def main():
     ap.add_argument("--rollouts", type=int, default=None)
     ap.add_argument("--timesteps", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed solve of each workload returned (U, baseline, normalizer, sum_w2) "
+                         "as DIR/<workload>_<array>.npy")
     ap.add_argument("--no-reference-gpu", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true",
                     help="default run only: skip the C2 / C3 / C5 summaries carried in the headline line (other_configs)")
